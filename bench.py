@@ -15,6 +15,8 @@ One step = one pass of the hot path over a batch of synthetic bodies.  Printed (
   roofline   HBM roofline of the translate pass: algorithmic bytes (input + output) ÷ CUDA-event duration vs MEASURED_PEAKS.json
   cpu_baseline  the oracle (CPU restatement of the reference Go path) on this box's host cores, bounded sample, rank 0 / N=1
 --impl reference times the CPU restatement alone on the same config (the reference is Go; no Go toolchain exists in the image).
+--dump-outputs DIR (config 2) writes what the device pass returned in its last timed step, a fixed seeded sample, as DIR/*.npy
+(float32 / float64, under 64 MB): with the same arguments the inputs are the same, so two builds can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -22,12 +24,14 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (no __pycache__ of the modules it imports)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -61,20 +65,21 @@ def batcher_block():
     aigw_batcher_translate with the bodies of the workload; callers, req/s and latency percentiles per setting."""
     try:
         import _workload as W
-        exe = "/tmp/aigw_batcher_load"
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-I", os.path.join(ROOT, "include"), os.path.join(ROOT, "tools", "batcher_load.cpp"), "-L", os.path.join(ROOT, "aigw_b200"),
-                               "-laigw_b200", "-Wl,-rpath," + os.path.join(ROOT, "aigw_b200"), "-lpthread", "-o", exe])
-        ar, of, le = W.chat_corpus(2, 0, 8000)
-        packed = b"".join(bytes(ar[int(of[i]):int(of[i]) + int(le[i])]) for i in range(8000))
-        po = np.zeros(8001, dtype=np.uint64); np.cumsum(le[:8000], out=po[1:])
-        open("/tmp/aigw_bl_bodies.bin", "wb").write(packed); open("/tmp/aigw_bl_offs.u64", "wb").write(po.tobytes())
-        rows = []
-        for threads, reqs, mb, win in ((1, 2000, 1, 0), (64, 1000, 64, 20), (256, 800, 256, 40), (512, 600, 512, 50)):
-            out = subprocess.check_output([exe, "/tmp/aigw_bl_bodies.bin", "/tmp/aigw_bl_offs.u64", "8000", str(threads), str(reqs), str(mb), str(win)], timeout=120).decode()
-            d = json.loads(out.strip().split("\n")[-1])
-            rows.append({"callers": threads, "max_batch": mb, "window_us": win, "req_per_s": d["requests_per_s"], "p50_us": d["p50_us"], "p99_us": d["p99_us"], "mean_batch": d["mean_batch"],
-                         "ok": d["ok"], "declined": d["declined"], "failed": d["failed"]})
-        return {"tool": "tools/batcher_load.cpp (closed loop: every caller submits its next request when the previous one returns)", "rows": rows}
+        with tempfile.TemporaryDirectory() as tmp:   # the tree may be read-only and fixed names under /tmp may belong to another user
+            exe, bodies_f, offs_f = (os.path.join(tmp, f) for f in ("aigw_batcher_load", "bodies.bin", "offs.u64"))
+            subprocess.check_call(["g++", "-O2", "-std=c++17", "-I", os.path.join(ROOT, "include"), os.path.join(ROOT, "tools", "batcher_load.cpp"), "-L", os.path.join(ROOT, "aigw_b200"),
+                                   "-laigw_b200", "-Wl,-rpath," + os.path.join(ROOT, "aigw_b200"), "-lpthread", "-o", exe])
+            ar, of, le = W.chat_corpus(2, 0, 8000)
+            packed = b"".join(bytes(ar[int(of[i]):int(of[i]) + int(le[i])]) for i in range(8000))
+            po = np.zeros(8001, dtype=np.uint64); np.cumsum(le[:8000], out=po[1:])
+            open(bodies_f, "wb").write(packed); open(offs_f, "wb").write(po.tobytes())
+            rows = []
+            for threads, reqs, mb, win in ((1, 2000, 1, 0), (64, 1000, 64, 20), (256, 800, 256, 40), (512, 600, 512, 50)):
+                out = subprocess.check_output([exe, bodies_f, offs_f, "8000", str(threads), str(reqs), str(mb), str(win)], timeout=120).decode()
+                d = json.loads(out.strip().split("\n")[-1])
+                rows.append({"callers": threads, "max_batch": mb, "window_us": win, "req_per_s": d["requests_per_s"], "p50_us": d["p50_us"], "p99_us": d["p99_us"], "mean_batch": d["mean_batch"],
+                             "ok": d["ok"], "declined": d["declined"], "failed": d["failed"]})
+            return {"tool": "tools/batcher_load.cpp (closed loop: every caller submits its next request when the previous one returns)", "rows": rows}
     except Exception as e:  # the bench line must not depend on a side tool
         return {"error": str(e)[:200]}
 
@@ -192,6 +197,34 @@ def escaped_corpus(arena, offs, lens, count):
     return out
 
 
+DUMP_ROWS = 65536          # result rows written by --dump-outputs (as float64: 5 MB)
+DUMP_OUT_BYTES = 8 << 20   # output bytes written by --dump-outputs (as float32: 32 MB)
+DUMP_FIELDS = ("status", "reason", "body_len", "path_len", "model_off", "model_len", "body_kind", "flags", "in_len")
+
+
+def dump_outputs(out_dir, ctx, res, d_out):
+    """--dump-outputs: what the last timed step of the device pass returned, on a fixed seeded sample of the bodies, so that two builds
+    can be compared output for output.  sample_index: the sampled bodies; result_<field>: their result rows (out_off is left out: where
+    a record lands in the output arena depends on the order the blocks claim space); output_bytes: the path + body bytes of the first
+    len(output_len) sampled bodies back to back, output_len[i] of them for the i-th (0 unless its status is OK)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(res)
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ROWS), replace=False))
+    rows = res[idx]
+    np.save(os.path.join(out_dir, "sample_index.npy"), idx.astype(np.float64))
+    for f in DUMP_FIELDS:
+        np.save(os.path.join(out_dir, f"result_{f}.npy"), rows[f].astype(np.float64))
+    rec = np.where(rows["status"] == 0, rows["path_len"].astype(np.int64) + rows["body_len"].astype(np.int64), 0)
+    m = int(np.searchsorted(np.cumsum(rec), DUMP_OUT_BYTES, side="right"))
+    out = np.zeros(int(rec[:m].sum()), dtype=np.uint8); o = 0
+    for r, l in zip(rows[:m], rec[:m]):
+        if l:
+            ctx.d2h(out[o:o + l], d_out + int(r["out_off"]))
+            o += int(l)
+    np.save(os.path.join(out_dir, "output_len.npy"), rec[:m].astype(np.float64))
+    np.save(os.path.join(out_dir, "output_bytes.npy"), out.astype(np.float32))
+
+
 def run_config2(a, rank, world, local, ncpu):
     import _oracle as O
     import _workload as W
@@ -254,6 +287,8 @@ def run_config2(a, rank, world, local, ncpu):
     wall = time.perf_counter() - t0
     dev_s = float(np.sum(kms)) / 1e3
     res = np.zeros(n, dtype=A.DocResult); ctx.d2h(res, d_res)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, ctx, res, d_out)
     n_ok = int((res["status"] == A.AIGW_OK).sum())
     out_bytes = int(res["body_len"].astype(np.uint64).sum() + res["path_len"].astype(np.uint64).sum())
     alg_bytes = int(lens.astype(np.uint64).sum()) + out_bytes  # SURVEY.md §8d: bytes_in + bytes_out per body
@@ -421,7 +456,7 @@ def run_config1(a, local, ncpu):
     from aigw_b200 import capi
     ra, ro, rl = capi.pack_bodies(resp)
     lat = []
-    for k in range(a.warmup + a.steps * 20):
+    for k in range(a.warmup + a.steps):
         t = time.perf_counter()
         res, out, st = ctx.chat_translate_host(cfg, pin, offs[:128].copy(), lens)
         ru = ctx.response_usage_host(ra, ro, rl)
@@ -711,7 +746,7 @@ def run_config5(a, rank, world, local, ncpu):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 5; config 1, where a step is one call and the line reports the median: 100)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--config", type=int, default=2, choices=[1, 2, 3, 4, 5])
     ap.add_argument("--bodies", type=int, default=int(os.environ.get("AIGW_BENCH_BODIES", 0)), help="bodies per GPU per step (config 2: 1,000,000; config 5: 1,250,000)")
@@ -722,7 +757,14 @@ def main():
     ap.add_argument("--skip-e2e", action="store_true")
     ap.add_argument("--e2e-lanes", type=int, default=1, help="config 2 e2e: host threads (each with its own context) keeping a call in flight; measured: 2 lanes x 8 sub-batches 4.81 M bodies/s vs 5.23 M for one call over the whole step (the call's own H2D / kernel / D2H pipeline is what counts)")
     ap.add_argument("--e2e-parts", type=int, default=1, help="config 2 e2e: sub-batches per step, dealt to the lanes round robin")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="config 2: write what the last timed step of the device pass returned (a fixed sample) to DIR/*.npy")
     a = ap.parse_args()
+    if a.steps is None:
+        a.steps = 100 if a.config == 1 and a.impl == "b200" else 5
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.config != 2):
+        ap.error("--dump-outputs is written by the device pass of config 2")
     rank = int(os.environ.get("RANK", 0)); world = int(os.environ.get("WORLD_SIZE", 1)); local = int(os.environ.get("LOCAL_RANK", 0))
     ncpu = host_cores()
     if a.bodies <= 0:

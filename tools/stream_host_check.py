@@ -5,8 +5,10 @@ import importlib.util
 import json
 import os
 import random
+import shutil
 import subprocess
 import sys
+import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests")); sys.path.insert(0, ROOT)
@@ -19,11 +21,20 @@ def load(name):
     spec = importlib.util.spec_from_file_location(name, os.path.join(ROOT, "tests", name + ".py")); m = importlib.util.module_from_spec(spec); spec.loader.exec_module(m); return m
 
 
+def cuda_include():
+    """include directory of the CUDA toolkit whose nvcc aigw_b200/build.py compiles with (None when there is none)"""
+    from aigw_b200.build import nvcc
+    exe = shutil.which(nvcc())
+    inc = os.path.join(os.path.dirname(os.path.dirname(os.path.realpath(exe))), "include") if exe else None
+    return inc if inc and os.path.exists(os.path.join(inc, "cuda_runtime.h")) else None
+
+
 class Host:
     def __init__(self):
-        exe = "/tmp/stream_host_check"
-        subprocess.check_call(["g++", "-O1", "-std=c++17", "-I/usr/local/cuda/include", "-o", exe, os.path.join(ROOT, "tools", "stream_host_check.cpp")], stderr=subprocess.DEVNULL)
-        self.p = subprocess.Popen([exe], stdin=subprocess.PIPE, stdout=subprocess.PIPE)
+        with tempfile.TemporaryDirectory() as d:   # a fixed name under /tmp may already belong to another user
+            exe = os.path.join(d, "stream_host_check")
+            subprocess.check_call(["g++", "-O1", "-std=c++17", "-I" + cuda_include(), "-o", exe, os.path.join(ROOT, "tools", "stream_host_check.cpp")], stderr=subprocess.DEVNULL)
+            self.p = subprocess.Popen([exe], stdin=subprocess.PIPE, stdout=subprocess.PIPE)
 
     def open(self, kind, model, response_id=b"", created=0):
         self.p.stdin.write(("open %d %s %s %d\n" % (KIND[kind], model.decode() or "-", response_id.decode() or "-", created)).encode())
