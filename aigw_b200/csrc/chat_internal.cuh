@@ -270,6 +270,6 @@ __host__ __device__ inline WorkPtrs carve(uint8_t* base, size_t ndocs, const Wor
 }
 
 // K2 (chat_walk.cu): validate + schema walk, one thread per document of the sub-batch
-cudaError_t launch_chat_walk(const ChatParams& P, uint32_t doc0, uint32_t ndocs, uint8_t* work, const WorkLayout& layout, cudaStream_t st, int blocks_per_sm = 0);   // 0: AIGW_WALK_BLOCKS
+cudaError_t launch_chat_walk(const ChatParams& P, uint32_t doc0, uint32_t ndocs, uint8_t* work, const WorkLayout& layout, cudaStream_t st);
 
 }  // namespace aigw

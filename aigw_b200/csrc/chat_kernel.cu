@@ -8,7 +8,6 @@
 //     reads from shared memory) and stored straight to the arena — no shared-memory image of the output.
 #include "chat_internal.cuh"
 
-#include <cstdlib>
 #include <mutex>
 
 #include "bulk.cuh"
@@ -24,9 +23,7 @@ namespace aigw {
 //   K2 walk    (thread per document)  stage 3+4 → jump table, copy ops, scratch, plan header
 //   K3 emit    (warp per document)    stage 5 → output record + result
 // K2 is where SIMT pays: 32 bodies with the same token count (≈ the same shape) share every instruction fetch.
-// Sub-batches are small enough for the bodies to stay in L2 between K1 and K3 (the body is read from DRAM once) and
-// alternate between two streams, so the latency-bound walk of one sub-batch runs under the issue-bound index / emit
-// of the other.
+// Sub-batches run one after the other on the caller's stream, each in the whole workspace.
 // ---- K1: structural index, one warp per document
 template <int MAXD, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32) chat_index_kernel(const __grid_constant__ ChatParams P, uint32_t doc0, uint32_t ndocs, uint8_t* work) {
@@ -220,17 +217,11 @@ size_t work_bytes_cls(size_t ndocs) { return work_per_doc(layout_of<MAXD>()) * n
 
 struct ClsConfig { bool ready = false; int bps1 = 1, bps3 = 1; };
 
-// documents per sub-batch: the bodies of the sub-batches in flight (two streams) stay in the 126 MB L2 between index and emit
-static size_t sub_batch_docs(int maxd) {
-  static const long env = getenv("AIGW_CHAT_SUB") ? atol(getenv("AIGW_CHAT_SUB")) : 0;
-  if (env > 0) return (size_t)env;
-  size_t d = ((size_t)40 << 20) / (size_t)maxd;
-  size_t p = 256; while (p * 2 <= d) p *= 2;
-  return p;
-}
+// the most documents one sub-batch takes (fewer when the workspace cannot hold that many)
+static constexpr size_t kSubBatchDocs = 262144;
 
 template <int MAXD, int WARPS>
-static cudaError_t launch_cls(const ChatParams& P, uint32_t first, int device, int sm_count, cudaStream_t st, uint8_t* work, size_t work_cap, const ChatAux* aux, cudaEvent_t* ev, int ev_cap,
+static cudaError_t launch_cls(const ChatParams& P, uint32_t first, int device, int sm_count, cudaStream_t st, uint8_t* work, size_t work_cap, cudaEvent_t* ev, int ev_cap,
                               int* launches) {
   using C = Cls<MAXD>;
   constexpr size_t hdr1 = (sizeof(IdTables) + 8 * WARPS + 15) & ~(size_t)15, hdr3 = (sizeof(LitTable::bytes) + 8 * WARPS + 15) & ~(size_t)15;
@@ -256,99 +247,29 @@ static cudaError_t launch_cls(const ChatParams& P, uint32_t first, int device, i
       cc.ready = true;
     }
   }
-  // stage timing (ev) needs the stages back to back on one stream; otherwise sub-batches rotate over the auxiliary streams
-  static const int env_streams = getenv("AIGW_CHAT_STREAMS") ? atoi(getenv("AIGW_CHAT_STREAMS")) : 1;   // > 1: sub-batches rotate over auxiliary streams
-  static const int env_idx_ctas = getenv("AIGW_IDX_CTAS") ? atoi(getenv("AIGW_IDX_CTAS")) : 0;      // experiments: cap resident CTAs per SM
-  static const int env_emit_ctas = getenv("AIGW_EMIT_CTAS") ? atoi(getenv("AIGW_EMIT_CTAS")) : 0;
-  static const int env_walk_ctas = getenv("AIGW_WALK_CTAS") ? atoi(getenv("AIGW_WALK_CTAS")) : 0;
-  static const int env_pipe = getenv("AIGW_CHAT_PIPE") ? atoi(getenv("AIGW_CHAT_PIPE")) : 0;
-  // ---- stage-pipelined mode: one stream per STAGE, sub-batches flow index -> walk -> emit through a ring of workspaces, so in
-  // the steady state one index, one walk and one emit kernel (of three consecutive sub-batches) are resident on every SM at
-  // once.  The walk is latency-bound (IPC 0.4) while index and emit are bound by the integer issue rate, so sharing an SM costs
-  // each little; every kernel's grid is capped so that the three fit together (registers: 3x128x80 + 2x128x54 + 2x128x56).
-  if (env_pipe && aux && !ev && P.n > 4096) {
-    const int ic = env_idx_ctas > 0 ? env_idx_ctas : 2, wc = env_walk_ctas > 0 ? env_walk_ctas : 3, ec = env_emit_ctas > 0 ? env_emit_ctas : 2;
-    const int bps1 = ic < cc.bps1 ? ic : cc.bps1, bps3 = ec < cc.bps3 ? ec : cc.bps3;
-    size_t sub = sub_batch_docs(MAXD);
-    int ring = kChatRing;
-    const size_t per = (chat_work_bytes(MAXD, sub) + 511) & ~(size_t)255;
-    while (ring > 1 && per * ring > work_cap) ring--;
-    if (per * ring > work_cap) { sub = (work_cap - kWorkHdr - 256) / work_per_doc(layout_of<MAXD>()); ring = 1; }
-    if (sub == 0) return cudaErrorMemoryAllocation;
-    cudaStream_t sI = aux->s[0], sW = aux->s[1], sE = aux->s[2];
-    cudaError_t e;
-    if ((e = cudaEventRecord(aux->fork, st)) != cudaSuccess) return e;
-    if ((e = cudaStreamWaitEvent(sI, aux->fork, 0)) != cudaSuccess) return e;
-    int nl = 0, sb = 0;
-    for (uint32_t rel = 0; rel < P.n; rel += (uint32_t)sub, sb++) {
-      const uint32_t doc0 = first + rel;
-      const uint32_t nd = (uint32_t)(P.n - rel < sub ? P.n - rel : sub);
-      const int slot = sb % ring;
-      uint8_t* wk = work + (size_t)slot * per;
-      const WorkPtrs wp = carve(wk, nd, layout_of<MAXD>());
-      long long want = ((long long)nd + WARPS - 1) / WARPS;
-      long long g1 = (long long)sm_count * bps1; if (want < g1) g1 = want;
-      long long g3 = (long long)sm_count * bps3; if (want < g3) g3 = want;
-      if (sb >= ring && (e = cudaStreamWaitEvent(sI, aux->emit_done[slot], 0)) != cudaSuccess) return e;   // the slot's previous tenant has been emitted
-      if ((e = cudaMemsetAsync(wk, 0, kWorkHdr, sI)) != cudaSuccess) return e;
-      chat_index_kernel<MAXD, WARPS><<<(unsigned)g1, WARPS * 32, smem1, sI>>>(P, doc0, nd, wk);
-      if ((e = cudaEventRecord(aux->idx_done[slot], sI)) != cudaSuccess) return e;
-      if ((e = cudaStreamWaitEvent(sW, aux->idx_done[slot], 0)) != cudaSuccess) return e;
-      { const unsigned gs = (nd + 8191) / 8192; chat_sort_kernel<<<gs < 32 ? gs : 32, kBins, 0, sW>>>(wp.ntok, wp.bins, wp.cursor, wp.perm, nd); }
-      if ((e = launch_chat_walk(P, doc0, nd, wk, layout_of<MAXD>(), sW, wc)) != cudaSuccess) return e;
-      if ((e = cudaEventRecord(aux->walk_done[slot], sW)) != cudaSuccess) return e;
-      if ((e = cudaStreamWaitEvent(sE, aux->walk_done[slot], 0)) != cudaSuccess) return e;
-      chat_emit_kernel<MAXD, WARPS><<<(unsigned)g3, WARPS * 32, smem3, sE>>>(P, doc0, nd, wk);
-      if ((e = cudaEventRecord(aux->emit_done[slot], sE)) != cudaSuccess) return e;
-      nl += 4;
-    }
-    // emits complete in order on sE, and every index / walk precedes its emit
-    if ((e = cudaEventRecord(aux->join[0], sE)) != cudaSuccess) return e;
-    if ((e = cudaStreamWaitEvent(st, aux->join[0], 0)) != cudaSuccess) return e;
-    if (launches) *launches = nl;
-    return cudaGetLastError();
-  }
-  const bool overlap = aux && !ev && P.n > 1024 && env_streams > 1;
-  const int nstreams = overlap ? (env_streams < kChatStreams ? env_streams : kChatStreams) : 1;
-  const size_t half = (work_cap / nstreams) & ~(size_t)255;
-  size_t sub = (half - kWorkHdr - 256) / work_per_doc(layout_of<MAXD>());
-  const size_t want_sub = overlap ? sub_batch_docs(MAXD) : 262144;
-  if (sub > want_sub) sub = want_sub;
+  size_t sub = ((work_cap & ~(size_t)255) - kWorkHdr - 256) / work_per_doc(layout_of<MAXD>());
+  if (sub > kSubBatchDocs) sub = kSubBatchDocs;
   if (sub == 0) return cudaErrorMemoryAllocation;
   cudaError_t e;
-  if (overlap) {
-    if ((e = cudaEventRecord(aux->fork, st)) != cudaSuccess) return e;
-    for (int s = 0; s < nstreams; s++) if ((e = cudaStreamWaitEvent(aux->s[s], aux->fork, 0)) != cudaSuccess) return e;
-  }
-  const int bps1 = overlap && env_idx_ctas > 0 && env_idx_ctas < cc.bps1 ? env_idx_ctas : cc.bps1;
-  const int bps3 = overlap && env_emit_ctas > 0 && env_emit_ctas < cc.bps3 ? env_emit_ctas : cc.bps3;
   int nl = 0, sb = 0;
   for (uint32_t rel = 0; rel < P.n; rel += (uint32_t)sub, sb++) {
     const uint32_t doc0 = first + rel;
     const uint32_t nd = (uint32_t)(P.n - rel < sub ? P.n - rel : sub);
-    cudaStream_t s = overlap ? aux->s[sb % nstreams] : st;
-    uint8_t* wk = work + (size_t)(overlap ? (sb % nstreams) : 0) * half;
-    const WorkPtrs wp = carve(wk, nd, layout_of<MAXD>());
-    if ((e = cudaMemsetAsync(wk, 0, kWorkHdr, s)) != cudaSuccess) return e;
+    const WorkPtrs wp = carve(work, nd, layout_of<MAXD>());
+    if ((e = cudaMemsetAsync(work, 0, kWorkHdr, st)) != cudaSuccess) return e;
     long long want = ((long long)nd + WARPS - 1) / WARPS;
-    long long g1 = (long long)sm_count * bps1; if (want < g1) g1 = want;
-    long long g3 = (long long)sm_count * bps3; if (want < g3) g3 = want;
+    long long g1 = (long long)sm_count * cc.bps1; if (want < g1) g1 = want;
+    long long g3 = (long long)sm_count * cc.bps3; if (want < g3) g3 = want;
     const bool timed = ev && 4 * sb + 3 < ev_cap;
-    if (timed) cudaEventRecord(ev[4 * sb + 0], s);
-    chat_index_kernel<MAXD, WARPS><<<(unsigned)g1, WARPS * 32, smem1, s>>>(P, doc0, nd, wk);
-    if (timed) cudaEventRecord(ev[4 * sb + 1], s);
-    { const unsigned gs = (nd + 8191) / 8192; chat_sort_kernel<<<gs < 32 ? gs : 32, kBins, 0, s>>>(wp.ntok, wp.bins, wp.cursor, wp.perm, nd); }
-    if ((e = launch_chat_walk(P, doc0, nd, wk, layout_of<MAXD>(), s, env_walk_ctas)) != cudaSuccess) return e;
-    if (timed) cudaEventRecord(ev[4 * sb + 2], s);
-    chat_emit_kernel<MAXD, WARPS><<<(unsigned)g3, WARPS * 32, smem3, s>>>(P, doc0, nd, wk);
-    if (timed) cudaEventRecord(ev[4 * sb + 3], s);
+    if (timed) cudaEventRecord(ev[4 * sb + 0], st);
+    chat_index_kernel<MAXD, WARPS><<<(unsigned)g1, WARPS * 32, smem1, st>>>(P, doc0, nd, work);
+    if (timed) cudaEventRecord(ev[4 * sb + 1], st);
+    { const unsigned gs = (nd + 8191) / 8192; chat_sort_kernel<<<gs < 32 ? gs : 32, kBins, 0, st>>>(wp.ntok, wp.bins, wp.cursor, wp.perm, nd); }
+    if ((e = launch_chat_walk(P, doc0, nd, work, layout_of<MAXD>(), st)) != cudaSuccess) return e;
+    if (timed) cudaEventRecord(ev[4 * sb + 2], st);
+    chat_emit_kernel<MAXD, WARPS><<<(unsigned)g3, WARPS * 32, smem3, st>>>(P, doc0, nd, work);
+    if (timed) cudaEventRecord(ev[4 * sb + 3], st);
     nl += 4;
-  }
-  if (overlap) {
-    for (int s = 0; s < nstreams; s++) {
-      if ((e = cudaEventRecord(aux->join[s], aux->s[s])) != cudaSuccess) return e;
-      if ((e = cudaStreamWaitEvent(st, aux->join[s], 0)) != cudaSuccess) return e;
-    }
   }
   if (launches) *launches = nl;
   return cudaGetLastError();
@@ -362,35 +283,23 @@ size_t chat_work_bytes(uint32_t max_len, size_t ndocs) {
   if (max_len <= 33792) return work_bytes_cls<33792>(ndocs);
   return work_bytes_cls<65536>(ndocs);
 }
-// workspace that lets a call of n documents run at full overlap: two sub-batches in flight
-size_t chat_work_bytes_for(uint32_t max_len, size_t n) {
-  static const int env_streams = getenv("AIGW_CHAT_STREAMS") ? atoi(getenv("AIGW_CHAT_STREAMS")) : 1;
-  static const int env_pipe = getenv("AIGW_CHAT_PIPE") ? atoi(getenv("AIGW_CHAT_PIPE")) : 0;
-  if (env_pipe && n > 4096) {
-    const int maxd = max_len <= 2048 ? 2048 : max_len <= 5120 ? 5120 : max_len <= 9216 ? 9216 : max_len <= 17408 ? 17408 : max_len <= 33792 ? 33792 : 65536;
-    return kChatRing * ((chat_work_bytes(maxd, sub_batch_docs(maxd)) + 511) & ~(size_t)255) + 512;
-  }
-  if (n <= 1024 || env_streams <= 1) return chat_work_bytes(max_len, n < 262144 ? n : 262144) + 512;
-  const int maxd = max_len <= 2048 ? 2048 : max_len <= 5120 ? 5120 : max_len <= 9216 ? 9216 : max_len <= 17408 ? 17408 : max_len <= 33792 ? 33792 : 65536;
-  size_t sub = sub_batch_docs(maxd);
-  if (sub > n) sub = n;
-  return kChatStreams * (chat_work_bytes(max_len, sub) + 512);
-}
+// workspace that lets a call of n documents run in one sub-batch, or in sub-batches of the largest size
+size_t chat_work_bytes_for(uint32_t max_len, size_t n) { return chat_work_bytes(max_len, n < kSubBatchDocs ? n : kSubBatchDocs) + 512; }
 
 cudaError_t launch_chat_translate_range(const ChatParams& P, uint32_t first, uint32_t count, uint32_t max_len, int device, int sm_count, cudaStream_t st, uint8_t* work, size_t work_cap,
-                                        const ChatAux* aux, int* launches) {
+                                        int* launches) {
   ChatParams Q = P; Q.n = count;
-  return launch_chat_translate(Q, max_len, device, sm_count, st, work, work_cap, aux, launches, nullptr, 0, first);
+  return launch_chat_translate(Q, max_len, device, sm_count, st, work, work_cap, launches, nullptr, 0, first);
 }
 
-cudaError_t launch_chat_translate(const ChatParams& P, uint32_t max_len, int device, int sm_count, cudaStream_t st, uint8_t* work, size_t work_cap, const ChatAux* aux, int* launches,
+cudaError_t launch_chat_translate(const ChatParams& P, uint32_t max_len, int device, int sm_count, cudaStream_t st, uint8_t* work, size_t work_cap, int* launches,
                                   cudaEvent_t* ev, int ev_cap, uint32_t first) {
-  if (max_len <= 2048) return launch_cls<2048, 4>(P, first, device, sm_count, st, work, work_cap, aux, ev, ev_cap, launches);
-  if (max_len <= 5120) return launch_cls<5120, 4>(P, first, device, sm_count, st, work, work_cap, aux, ev, ev_cap, launches);
-  if (max_len <= 9216) return launch_cls<9216, 2>(P, first, device, sm_count, st, work, work_cap, aux, ev, ev_cap, launches);
-  if (max_len <= 17408) return launch_cls<17408, 2>(P, first, device, sm_count, st, work, work_cap, aux, ev, ev_cap, launches);
-  if (max_len <= 33792) return launch_cls<33792, 1>(P, first, device, sm_count, st, work, work_cap, aux, ev, ev_cap, launches);
-  return launch_cls<65536, 1>(P, first, device, sm_count, st, work, work_cap, aux, ev, ev_cap, launches);
+  if (max_len <= 2048) return launch_cls<2048, 4>(P, first, device, sm_count, st, work, work_cap, ev, ev_cap, launches);
+  if (max_len <= 5120) return launch_cls<5120, 4>(P, first, device, sm_count, st, work, work_cap, ev, ev_cap, launches);
+  if (max_len <= 9216) return launch_cls<9216, 2>(P, first, device, sm_count, st, work, work_cap, ev, ev_cap, launches);
+  if (max_len <= 17408) return launch_cls<17408, 2>(P, first, device, sm_count, st, work, work_cap, ev, ev_cap, launches);
+  if (max_len <= 33792) return launch_cls<33792, 1>(P, first, device, sm_count, st, work, work_cap, ev, ev_cap, launches);
+  return launch_cls<65536, 1>(P, first, device, sm_count, st, work, work_cap, ev, ev_cap, launches);
 }
 
 }  // namespace aigw

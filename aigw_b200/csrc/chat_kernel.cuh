@@ -286,23 +286,21 @@ struct Cls {
 };
 
 // Workspace: chat_work_bytes(max_len, docs_per_sub_batch) bytes hold one sub-batch of intermediates; the launcher walks P.n
-// documents in sub-batches (4 launches each).  With `aux` (two extra streams + events, owned by the context) consecutive
-// sub-batches alternate between the two streams and two halves of the workspace: chat_work_bytes_for(max_len, n) is the size
-// that lets a call of n documents do so.  `stage_events` (profiling) forces one stream with the stages back to back.
+// documents in sub-batches of at most 256 Ki documents (4 launches each), one after the other on the caller's stream, each
+// reusing the whole workspace.  chat_work_bytes_for(max_len, n) is the size that holds the largest sub-batch a call of n
+// documents needs.  `stage_events` (profiling) receives four events per sub-batch at the stage boundaries (before index,
+// after index, after sort + walk, after emit) for the first stage_event_cap / 4 sub-batches.
 // Per-device kernel attributes are configured on first use of each (device, size class).
 static constexpr int kMaxDevices = 16;
-static constexpr int kChatStreams = 4;
-static constexpr int kChatRing = 4;   // sub-batch workspaces in flight in the stage-pipelined mode
-struct ChatAux { cudaStream_t s[kChatStreams]; cudaEvent_t fork, join[kChatStreams], idx_done[kChatRing], walk_done[kChatRing], emit_done[kChatRing]; };
 static constexpr uint32_t kSmallMaxLen = 5120;   // the fused small-batch kernel's size class
 // fused index + walk + emit, one CTA per document; out_slot[i] .. out_slot[i+1] is document i's output slot in P.out; no workspace
 cudaError_t launch_chat_small(const ChatParams& P, uint32_t doc0, uint32_t ndocs, const uint64_t* out_slot, cudaStream_t st);
 size_t chat_work_bytes(uint32_t max_len, size_t ndocs);
 size_t chat_work_bytes_for(uint32_t max_len, size_t n);
-cudaError_t launch_chat_translate(const ChatParams& P, uint32_t max_len, int device, int sm_count, cudaStream_t st, uint8_t* work, size_t work_cap, const ChatAux* aux, int* launches,
+cudaError_t launch_chat_translate(const ChatParams& P, uint32_t max_len, int device, int sm_count, cudaStream_t st, uint8_t* work, size_t work_cap, int* launches,
                                   cudaEvent_t* stage_events, int stage_event_cap, uint32_t first = 0);
 // documents [first, first+count): offsets / lens / results are indexed with the global document number
 cudaError_t launch_chat_translate_range(const ChatParams& P, uint32_t first, uint32_t count, uint32_t max_len, int device, int sm_count, cudaStream_t st, uint8_t* work,
-                                        size_t work_cap, const ChatAux* aux, int* launches);
+                                        size_t work_cap, int* launches);
 
 }  // namespace aigw

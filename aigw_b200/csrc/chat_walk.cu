@@ -1,8 +1,6 @@
 // K2 launcher: picks the walk kernel of the schema's group (chat_walk_g*.cu, one translation unit per group).
 #include "chat_internal.cuh"
 
-#include <cstdlib>
-
 namespace aigw {
 
 #define AIGW_WALK_DECL(g) cudaError_t launch_chat_walk_g##g(const ChatParams&, uint32_t, uint32_t, uint8_t*, const WorkLayout&, cudaStream_t, int);
@@ -12,13 +10,11 @@ AIGW_WALK_DECL(0) AIGW_WALK_DECL(1) AIGW_WALK_DECL(2) AIGW_WALK_DECL(3) AIGW_WAL
 AIGW_SMALL_DECL(0) AIGW_SMALL_DECL(1) AIGW_SMALL_DECL(2) AIGW_SMALL_DECL(3) AIGW_SMALL_DECL(4) AIGW_SMALL_DECL(5) AIGW_SMALL_DECL(6) AIGW_SMALL_DECL(7) AIGW_SMALL_DECL(8) AIGW_SMALL_DECL(9)
 #undef AIGW_SMALL_DECL
 
-cudaError_t launch_chat_walk(const ChatParams& P, uint32_t doc0, uint32_t ndocs, uint8_t* work, const WorkLayout& layout, cudaStream_t st, int blocks_per_sm) {
+cudaError_t launch_chat_walk(const ChatParams& P, uint32_t doc0, uint32_t ndocs, uint8_t* work, const WorkLayout& layout, cudaStream_t st) {
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   { static int sm_cache[kMaxDevices] = {0}; if (dev >= 0 && dev < kMaxDevices) { if (!sm_cache[dev]) cudaDeviceGetAttribute(&sm_cache[dev], cudaDevAttrMultiProcessorCount, dev); sms = sm_cache[dev] ? sm_cache[dev] : 148; } }
-  static const int env_ctas = getenv("AIGW_WALK_CTAS") ? atoi(getenv("AIGW_WALK_CTAS")) : 0;   // experiment: fewer resident blocks per SM (room for the other stages' blocks)
-  if (blocks_per_sm <= 0 || blocks_per_sm > AIGW_WALK_BLOCKS) blocks_per_sm = env_ctas > 0 && env_ctas < AIGW_WALK_BLOCKS ? env_ctas : AIGW_WALK_BLOCKS;
-  sms *= blocks_per_sm;
+  sms *= AIGW_WALK_BLOCKS;
   const uint32_t s = P.schema;
   if (s & (uint32_t)AIGW_SCHEMA_MESSAGES)   // the full re-maps (OpenAI / Bedrock targets) have their own kernel
     return ((s & 15u) == (uint32_t)AIGW_SCHEMA_OPENAI || (s & 15u) == (uint32_t)AIGW_SCHEMA_AWS_BEDROCK) ? launch_chat_walk_g9(P, doc0, ndocs, work, layout, st, sms) : launch_chat_walk_g7(P, doc0, ndocs, work, layout, st, sms);

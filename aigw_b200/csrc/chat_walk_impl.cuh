@@ -2925,17 +2925,14 @@ __global__ void __launch_bounds__(32) AIGW_CAT(chat_small_kernel_g, AIGW_WALK_GR
     if (lane == 0) P.results[doc] = res;
     return;
   }
-  const long long t0 = clock64();
   // body (the loads of the whole body are in flight together: one PCIe round trip when the buffer is mapped host memory), literals
   if ((reinterpret_cast<uintptr_t>(g) & 15u) == 0) { const uint4* g4 = (const uint4*)g; uint4* d4 = (uint4*)s_in; for (uint32_t i = lane; i < (len + 15u) >> 4; i += 32) d4[i] = g4[i]; }
   else for (uint32_t i = lane; i < len; i += 32) s_in[i] = g[i];
   { const uint4* l4 = (const uint4*)g_small_lits.bytes; uint4* d4 = (uint4*)s_lits; for (uint32_t i = lane; i < S::kLits / 16; i += 32) d4[i] = l4[i]; }
   __syncwarp();
   const IdTables* ids = (P.schema & AIGW_SCHEMA_MESSAGES) ? &g_small_ids_msg : (P.schema & 48) == AIGW_SCHEMA_RESP_AWS_BEDROCK ? &g_small_ids_resp : &g_small_ids;
-  const long long t1 = clock64();
   const uint32_t ntok = index_doc<MAXD>(s_in, len, lane, s_tw, s_bs, s_nc, ids);
   __syncwarp();
-  const long long t2 = clock64();
   if (lane == 0) {
     WalkBufs B;
     B.body = s_in; B.len = len; B.tw = s_tw; B.jmp = s_jmp; B.ops = s_ops; B.scr = s_scr;
@@ -2944,7 +2941,6 @@ __global__ void __launch_bounds__(32) AIGW_CAT(chat_small_kernel_g, AIGW_WALK_GR
     *s_po = pw;
   }
   __syncwarp();
-  const long long t3 = clock64();
   const PlanOut po = *s_po;
   if (po.reason) {
     res.reason = po.reason;
@@ -2967,7 +2963,6 @@ __global__ void __launch_bounds__(32) AIGW_CAT(chat_small_kernel_g, AIGW_WALK_GR
     res.out_off = obase + P.out_bias; res.body_len = olen - po.path_len; res.path_len = (uint16_t)po.path_len; res.status = AIGW_OK; res.reason = 0;
     res.model_off = po.model_off; res.model_len = po.model_len; res.body_kind = (po.flags & 0x80u) ? AIGW_BODY_UNCHANGED : AIGW_BODY_BYTES; res.flags = po.flags & 0x7fu;
     P.results[doc] = res;
-    if (P.next_doc && li == 0) { const long long t4 = clock64(); P.next_doc[0] = (unsigned)(t1 - t0); P.next_doc[1] = (unsigned)(t2 - t1); P.next_doc[2] = (unsigned)(t3 - t2); P.next_doc[3] = (unsigned)(t4 - t3); }   // phase clocks (debug)
   }
 }
 

@@ -2,7 +2,6 @@
 // The host path is a 3-slot pipeline: H2D(chunk c+1) ‖ kernel(chunk c) ‖ D2H(chunk c-1) on three
 // CUDA streams; everything computed is computed by the kernels in this directory — there is no
 // CPU fallback anywhere in this library.
-#include <chrono>
 #include <cstdio>
 #include <sched.h>
 #include <cstdlib>
@@ -40,10 +39,7 @@ struct ChunkSlot {
   uint32_t* d_map = nullptr; size_t map_cap = 0;   // size-class bucketing: documents of the chunk grouped by class
   uint8_t* d_out = nullptr; size_t out_cap = 0;
   aigw_doc_result* d_res = nullptr;
-  unsigned long long* d_used = nullptr;   // device bump counter
-  unsigned int* d_next = nullptr;         // device work counter
-  unsigned long long* h_used = nullptr;   // pinned mirror
-  cudaEvent_t ev_h2d, ev_k0, ev_k1, ev_ctr, ev_done;
+  cudaEvent_t ev_h2d, ev_k1, ev_done;
 };
 
 struct aigw_bpe { uint2* d_table = nullptr; uint16_t* d_b2i = nullptr; uint32_t slots = 0; };
@@ -59,7 +55,7 @@ struct aigw_ctx {
   // host-API output (pinned)
   uint8_t* h_out = nullptr; size_t h_out_cap = 0;
   aigw_doc_result* h_res = nullptr; size_t h_res_cap = 0;
-  long small_max = -1;   // aigw_chat_set_small_batch; -1: AIGW_SMALL_MAX or 512
+  long small_max = -1;   // aigw_chat_set_small_batch; -1: 512
   // BPE count (host form): device staging
   uint8_t* d_bpe_text = nullptr; size_t bpe_text_cap = 0; uint64_t* d_bpe_off = nullptr; size_t bpe_off_cap = 0; uint32_t* d_bpe_len = nullptr; size_t bpe_len_cap = 0; uint32_t* d_bpe_cnt = nullptr; size_t bpe_cnt_cap = 0;
   // large embeddings requests (aigw_embeddings_count_*): token workspace, text table, counts, host-form staging
@@ -71,8 +67,7 @@ struct aigw_ctx {
   uint8_t* d_work = nullptr; size_t work_cap = 0;
   unsigned long long* d_used_arr = nullptr; unsigned long long* h_used_arr = nullptr; size_t used_cap = 0;  // per-chunk bump counters
   cudaEvent_t stage_ev[64]; float stage_ms[3] = {0, 0, 0}; int last_launches = 0;
-  bool profile_stages = false;   // aigw_chat_set_profile: next device calls run the stages back to back on one stream and time them
-  ChatAux aux{};                 // two extra streams: sub-batches of one call alternate between them
+  bool profile_stages = false;   // aigw_chat_set_profile: next device calls time the stages
   // sse host-API device buffers
   uint8_t* d_sse_bytes = nullptr; size_t sse_bytes_cap = 0;
   uint64_t* d_sse_coff = nullptr; size_t sse_coff_cap = 0;
@@ -155,8 +150,8 @@ cudaError_t chat_small_launch(const aigw_backend_cfg* cfg, const uint8_t* in, co
 // host loops over the calls of one window (byte staging, result hand-back) run on a few threads when the window is large
 template <class F>
 static void host_parallel_for(uint32_t n, F&& f) {
-  static const unsigned hw = [] { unsigned h = 2; const char* e = getenv("AIGW_HOST_THREADS"); if (e) h = (unsigned)atoi(e); return h < 1 ? 1u : (h > 8 ? 8u : h); }();   // measured: more staging threads slow the DMA that follows (17.3 / 20.0 / 19.5 / 15.9 M chunks/s at 1 / 2 / 4 / 8)
-  if (n < 16384 || hw == 1) { f(0u, n); return; }
+  constexpr unsigned hw = 2;   // measured: more staging threads slow the DMA that follows (17.3 / 20.0 / 19.5 / 15.9 M chunks/s at 1 / 2 / 4 / 8)
+  if (n < 16384) { f(0u, n); return; }
   std::vector<std::thread> th;
   const uint32_t per = (n + hw - 1) / hw;
   for (unsigned t = 1; t < hw; t++) { const uint32_t b = t * per, e = b + per < n ? b + per : n; if (b < e) th.emplace_back([&f, b, e] { f(b, e); }); }
@@ -187,16 +182,11 @@ int aigw_init(int device, aigw_ctx** out) {
   INIT_CK(cudaStreamCreateWithFlags(&ctx->s_compute, cudaStreamNonBlocking));
   INIT_CK(cudaStreamCreateWithFlags(&ctx->s_h2d, cudaStreamNonBlocking));
   INIT_CK(cudaStreamCreateWithFlags(&ctx->s_d2h, cudaStreamNonBlocking));
-  for (int k = 0; k < kChatStreams; k++) { INIT_CK(cudaStreamCreateWithFlags(&ctx->aux.s[k], cudaStreamNonBlocking)); INIT_CK(cudaEventCreateWithFlags(&ctx->aux.join[k], cudaEventDisableTiming)); }
-  INIT_CK(cudaEventCreateWithFlags(&ctx->aux.fork, cudaEventDisableTiming));
-  for (int k = 0; k < kChatRing; k++) { INIT_CK(cudaEventCreateWithFlags(&ctx->aux.idx_done[k], cudaEventDisableTiming)); INIT_CK(cudaEventCreateWithFlags(&ctx->aux.walk_done[k], cudaEventDisableTiming)); INIT_CK(cudaEventCreateWithFlags(&ctx->aux.emit_done[k], cudaEventDisableTiming)); }
   INIT_CK(cudaMalloc(&ctx->d_counters, 256 * sizeof(unsigned int)));
   INIT_CK(cudaEventCreate(&ctx->ev0)); INIT_CK(cudaEventCreate(&ctx->ev1));
   for (auto& e2 : ctx->stage_ev) INIT_CK(cudaEventCreate(&e2));
   for (auto& s : ctx->slot) {
-    INIT_CK(cudaEventCreateWithFlags(&s.ev_h2d, cudaEventDisableTiming)); INIT_CK(cudaEventCreate(&s.ev_k0)); INIT_CK(cudaEventCreate(&s.ev_k1));
-    INIT_CK(cudaEventCreateWithFlags(&s.ev_ctr, cudaEventDisableTiming)); INIT_CK(cudaEventCreateWithFlags(&s.ev_done, cudaEventDisableTiming));
-    INIT_CK(cudaMalloc(&s.d_used, 8)); INIT_CK(cudaMalloc(&s.d_next, 4)); INIT_CK(cudaHostAlloc(&s.h_used, 8, cudaHostAllocDefault));
+    INIT_CK(cudaEventCreateWithFlags(&s.ev_h2d, cudaEventDisableTiming)); INIT_CK(cudaEventCreate(&s.ev_k1)); INIT_CK(cudaEventCreateWithFlags(&s.ev_done, cudaEventDisableTiming));
   }
 #undef INIT_CK
   *out = ctx;
@@ -208,8 +198,8 @@ void aigw_destroy(aigw_ctx* ctx) {
   cudaSetDevice(ctx->device);
   cudaDeviceSynchronize();
   for (auto& s : ctx->slot) {
-    cudaFree(s.d_in); cudaFree(s.d_off); cudaFree(s.d_len); cudaFree(s.d_out); cudaFree(s.d_res); cudaFree(s.d_used); cudaFree(s.d_next); cudaFreeHost(s.h_used);
-    cudaEventDestroy(s.ev_h2d); cudaEventDestroy(s.ev_k0); cudaEventDestroy(s.ev_k1); cudaEventDestroy(s.ev_ctr); cudaEventDestroy(s.ev_done);
+    cudaFree(s.d_in); cudaFree(s.d_off); cudaFree(s.d_len); cudaFree(s.d_map); cudaFree(s.d_out); cudaFree(s.d_res);
+    cudaEventDestroy(s.ev_h2d); cudaEventDestroy(s.ev_k1); cudaEventDestroy(s.ev_done);
   }
   cudaFreeHost(ctx->h_out); cudaFreeHost(ctx->h_res); cudaFreeHost(ctx->h_small); cudaFree(ctx->d_bpe_text); cudaFree(ctx->d_bpe_off); cudaFree(ctx->d_bpe_len); cudaFree(ctx->d_bpe_cnt); cudaFree(ctx->d_emb_tok); cudaFree(ctx->d_emb_toff); cudaFree(ctx->d_emb_tlen); cudaFree(ctx->d_emb_cnt); cudaFree(ctx->d_emb_body); cudaFree(ctx->d_emb_off); cudaFree(ctx->d_emb_len); cudaFree(ctx->d_emb_res); cudaFree(ctx->d_counters); cudaFree(ctx->d_work); cudaFree(ctx->d_used_arr); cudaFreeHost(ctx->h_used_arr);
   for (auto& e2 : ctx->stage_ev) cudaEventDestroy(e2);
@@ -221,9 +211,6 @@ void aigw_destroy(aigw_ctx* ctx) {
     cudaFree(sp.d_slots); cudaFreeHost(sp.h_in); cudaFree(sp.d_in); cudaFreeHost(sp.h_steps); cudaFree(sp.d_steps); cudaFree(sp.d_res); cudaFreeHost(sp.h_res);
     cudaFree(sp.d_out); cudaFree(sp.d_packed); cudaFreeHost(sp.h_packed); cudaFree(sp.d_used); cudaFreeHost(sp.h_used); cudaFree(sp.d_tmpl); cudaFree(sp.d_ids); cudaFreeHost(sp.h_ids);
   }
-  for (int k = 0; k < kChatStreams; k++) { if (ctx->aux.s[k]) cudaStreamDestroy(ctx->aux.s[k]); if (ctx->aux.join[k]) cudaEventDestroy(ctx->aux.join[k]); }
-  if (ctx->aux.fork) cudaEventDestroy(ctx->aux.fork);
-  for (int k = 0; k < kChatRing; k++) { if (ctx->aux.idx_done[k]) cudaEventDestroy(ctx->aux.idx_done[k]); if (ctx->aux.walk_done[k]) cudaEventDestroy(ctx->aux.walk_done[k]); if (ctx->aux.emit_done[k]) cudaEventDestroy(ctx->aux.emit_done[k]); }
   delete ctx;
 }
 
@@ -280,14 +267,14 @@ static int chat_translate_device_impl(aigw_ctx* ctx, const aigw_backend_cfg* cfg
   uint32_t ml = max_len ? max_len : 65536u;
   if (cfg && (cfg->schema & 48) == AIGW_SCHEMA_RESP_AWS_BEDROCK) ml = resp_class_len(ml);
   const bool stages = ctx->profile_stages && kernel_ms;
-  {  // workspace: two sub-batches in flight (one per auxiliary stream); profiling runs one large sub-batch at a time
+  {  // workspace: one sub-batch of intermediates
     size_t need = chat_work_bytes_for(ml, n);
     const size_t cap = (size_t)3 << 30, floor1 = chat_work_bytes(ml, 1024);
     if (need > cap) need = cap > floor1 ? cap : floor1;
     ENSURE(ctx->d_work, ctx->work_cap, need, false);
   }
   if (kernel_ms) CK(cudaEventRecord(ctx->ev0, st));
-  CK(launch_chat_translate(P, ml, ctx->device, ctx->sm_count, st, ctx->d_work, ctx->work_cap, &ctx->aux, &ctx->last_launches, stages ? ctx->stage_ev : nullptr, 64, first));
+  CK(launch_chat_translate(P, ml, ctx->device, ctx->sm_count, st, ctx->d_work, ctx->work_cap, &ctx->last_launches, stages ? ctx->stage_ev : nullptr, 64, first));
   if (kernel_ms) {
     CK(cudaEventRecord(ctx->ev1, st)); CK(cudaEventSynchronize(ctx->ev1)); CK(cudaEventElapsedTime(kernel_ms, ctx->ev0, ctx->ev1));
     if (stages) {
@@ -345,15 +332,11 @@ static int chat_small_host(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const uin
   ChatParams P; fill_params(P, cfg);
   P.bodies = d_small + tab; P.offsets = (const uint64_t*)d_small; P.lens = (const uint32_t*)(d_small + ((size_t)n + 1) * 16); P.n = n;
   P.out = d_out; P.out_capacity = so; P.results = d_res; P.out_used = nullptr; P.next_doc = nullptr; P.out_bias = 0; P.doc_map = nullptr;
-  static const bool dbg = getenv("AIGW_SMALL_DBG") != nullptr;
-  static unsigned int* h_dbg = nullptr;
-  if (dbg) { if (!h_dbg) cudaHostAlloc((void**)&h_dbg, 64, cudaHostAllocDefault); P.next_doc = h_dbg; }
   CK(cudaEventRecord(ctx->ev0, ctx->s_compute));
   CK(launch_chat_small(P, 0, n, (const uint64_t*)d_small + n + 1, ctx->s_compute));
   CK(cudaEventRecord(ctx->ev1, ctx->s_compute));
   CK(cudaEventSynchronize(ctx->ev1));
   float kms = 0; cudaEventElapsedTime(&kms, ctx->ev0, ctx->ev1);
-  if (dbg) fprintf(stderr, "small n=%u kernel %.1f us  clocks: load %u index %u walk %u emit %u\n", n, kms * 1e3f, h_dbg[0], h_dbg[1], h_dbg[2], h_dbg[3]);
   uint64_t produced = 0;
   for (uint32_t i = 0; i < n; i++) if (ctx->h_res[i].status == AIGW_OK) produced += ((uint64_t)ctx->h_res[i].path_len + ctx->h_res[i].body_len + 15u) & ~15ull;
   out->results = ctx->h_res; out->out = ctx->h_out; out->out_used = so; out->h2d_bytes = in_bytes + tab; out->d2h_bytes = produced + (uint64_t)n * sizeof(aigw_doc_result);
@@ -370,20 +353,15 @@ int aigw_chat_translate_host(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const u
   //   SMs             index / sort / walk / emit of chunk c → device (s_compute)
   //   copy engine B   D2H of chunk c-1: exactly the bytes the emit stage produced + the chunk's result table (s_d2h)
   // The host runs one chunk behind the GPU (it waits for chunk c-1's byte count while chunk c's kernels are queued).
-  // AIGW_HOST_ZEROCOPY=1 restores the round-1 variant (emit stores straight into mapped host memory) for A/B runs.
   memset(out, 0, sizeof *out);
   if (n == 0) return 0;
   CK(cudaSetDevice(ctx->device));
-  {
-    static const long env_small_max = getenv("AIGW_SMALL_MAX") ? atol(getenv("AIGW_SMALL_MAX")) : 512;   // 0 disables the fused small-batch path
-    if ((long)n <= (ctx->small_max >= 0 ? ctx->small_max : env_small_max)) {
-      const bool resp = cfg && (cfg->schema & 48) == AIGW_SCHEMA_RESP_AWS_BEDROCK;
-      uint32_t ml = 0; for (uint32_t i = 0; i < n; i++) if (lens[i] > ml) ml = lens[i];
-      if ((resp ? resp_class_len(ml) : ml) <= kSmallMaxLen) return chat_small_host(ctx, cfg, bodies, offsets, lens, n, out);
-    }
+  if ((long)n <= (ctx->small_max >= 0 ? ctx->small_max : 512)) {   // 0 disables the fused small-batch path
+    const bool resp = cfg && (cfg->schema & 48) == AIGW_SCHEMA_RESP_AWS_BEDROCK;
+    uint32_t ml = 0; for (uint32_t i = 0; i < n; i++) if (lens[i] > ml) ml = lens[i];
+    if ((resp ? resp_class_len(ml) : ml) <= kSmallMaxLen) return chat_small_host(ctx, cfg, bodies, offsets, lens, n, out);
   }
-  static const bool zero_copy = getenv("AIGW_HOST_ZEROCOPY") != nullptr;
-  static const uint64_t kChunkBytes = (uint64_t)(getenv("AIGW_CHUNK_MB") ? atol(getenv("AIGW_CHUNK_MB")) : 256) << 20;   // pipeline granularity (fill / drain cost vs per-chunk launches)
+  constexpr uint64_t kChunkBytes = 256ull << 20;   // pipeline granularity (fill / drain cost vs per-chunk launches)
   std::vector<uint32_t> cb;  // chunk begin doc index
   cb.push_back(0);
   uint32_t max_len = 0;
@@ -412,7 +390,7 @@ int aigw_chat_translate_host(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const u
   for (int s = 0; s < nslots; s++) {
     ChunkSlot& S = ctx->slot[s];
     ENSURE(S.d_in, S.in_cap, max_in + 64, false);
-    if (!zero_copy) { ENSURE(S.d_out, S.out_cap, max_out + 64, false); }
+    ENSURE(S.d_out, S.out_cap, max_out + 64, false);
     if (S.doc_cap < max_docs) {
       cudaFree(S.d_off); cudaFree(S.d_len); cudaFree(S.d_res); S.doc_cap = 0;
       const size_t dc = max_docs + max_docs / 8 + 16;
@@ -440,8 +418,6 @@ int aigw_chat_translate_host(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const u
     CK(cudaMalloc(&ctx->d_used_arr, cap * 8)); CK(cudaHostAlloc(&ctx->h_used_arr, cap * 8, cudaHostAllocDefault));
     ctx->used_cap = cap;
   }
-  uint8_t* dev_out = nullptr; aigw_doc_result* dev_res = nullptr;  // device views of the pinned arenas (zero-copy variant)
-  if (zero_copy) { CK(cudaHostGetDevicePointer((void**)&dev_out, ctx->h_out, 0)); CK(cudaHostGetDevicePointer((void**)&dev_res, ctx->h_res, 0)); }
 
   ChatParams P0; fill_params(P0, cfg);
   uint64_t h2d = 0, d2h = (uint64_t)n * sizeof(aigw_doc_result) + (uint64_t)nch * 8;
@@ -452,12 +428,10 @@ int aigw_chat_translate_host(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const u
     CK(cudaEventSynchronize(S.ev_k1));
     const uint64_t used = ctx->h_used_arr[k] < out_cap[k] ? ctx->h_used_arr[k] : out_cap[k];
     d2h += used;
-    if (!zero_copy) {
-      const uint32_t b = cb[k], nd = cb[k + 1] - b;
-      if (used) CK(cudaMemcpyAsync(ctx->h_out + out_base[k], S.d_out, used, cudaMemcpyDeviceToHost, ctx->s_d2h));
-      CK(cudaMemcpyAsync(ctx->h_res + b, S.d_res, (size_t)nd * sizeof(aigw_doc_result), cudaMemcpyDeviceToHost, ctx->s_d2h));
-      CK(cudaEventRecord(S.ev_done, ctx->s_d2h));
-    }
+    const uint32_t b = cb[k], nd = cb[k + 1] - b;
+    if (used) CK(cudaMemcpyAsync(ctx->h_out + out_base[k], S.d_out, used, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(ctx->h_res + b, S.d_res, (size_t)nd * sizeof(aigw_doc_result), cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaEventRecord(S.ev_done, ctx->s_d2h));
     return 0;
   };
   for (int c = 0; c < nch; c++) {
@@ -465,7 +439,7 @@ int aigw_chat_translate_host(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const u
     const uint32_t b = cb[c], e = cb[c + 1], nd = e - b;
     if (c >= nslots) {
       CK(cudaStreamWaitEvent(ctx->s_h2d, S.ev_k1, 0));                       // the slot's input has been consumed
-      if (!zero_copy) CK(cudaStreamWaitEvent(ctx->s_compute, S.ev_done, 0));   // the slot's output has left the device
+      CK(cudaStreamWaitEvent(ctx->s_compute, S.ev_done, 0));                 // the slot's output has left the device
     }
     CK(cudaMemcpyAsync(S.d_in, bodies + offsets[b], in_bytes[c] - 16, cudaMemcpyHostToDevice, ctx->s_h2d));
     CK(cudaMemcpyAsync(S.d_off, offsets + b, (size_t)nd * 8, cudaMemcpyHostToDevice, ctx->s_h2d));
@@ -475,8 +449,6 @@ int aigw_chat_translate_host(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const u
     uint32_t cls_cnt[6] = {0, 0, 0, 0, 0, 0};
     for (uint32_t i = b; i < e; i++) cls_cnt[cls_of(lens[i])]++;
     int n_cls = 0, top_cls = 0; for (int k = 0; k < 6; k++) if (cls_cnt[k]) { n_cls++; top_cls = k; }
-    static const bool no_bucketing = getenv("AIGW_NO_BUCKETING") != nullptr;   // A/B switch for the Zipf bench
-    if (no_bucketing) n_cls = 1;
     uint32_t cls_start[7] = {0, 0, 0, 0, 0, 0, 0};
     if (n_cls > 1) {
       for (int k = 0; k < 6; k++) cls_start[k + 1] = cls_start[k] + cls_cnt[k];
@@ -493,19 +465,19 @@ int aigw_chat_translate_host(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const u
     ChatParams P = P0;
     P.bodies = S.d_in - offsets[b];  // absolute offsets index straight into the chunk
     P.offsets = S.d_off - b; P.lens = S.d_len - b; P.n = nd;
-    P.out = zero_copy ? dev_out + out_base[c] : S.d_out; P.out_capacity = out_cap[c];
-    P.results = zero_copy ? dev_res : S.d_res - b; P.out_used = ctx->d_used_arr + c; P.next_doc = nullptr; P.out_bias = out_base[c]; P.doc_map = nullptr;
+    P.out = S.d_out; P.out_capacity = out_cap[c];
+    P.results = S.d_res - b; P.out_used = ctx->d_used_arr + c; P.next_doc = nullptr; P.out_bias = out_base[c]; P.doc_map = nullptr;
     // documents keep their global index: kernels address offsets/lens/results with doc0 + i (or doc_map[i])
     if (n_cls <= 1) {
       int nl = 0;
-      CK(launch_chat_translate_range(P, b, nd, kClsMax[top_cls], ctx->device, ctx->sm_count, ctx->s_compute, ctx->d_work, ctx->work_cap, &ctx->aux, &nl));
+      CK(launch_chat_translate_range(P, b, nd, kClsMax[top_cls], ctx->device, ctx->sm_count, ctx->s_compute, ctx->d_work, ctx->work_cap, &nl));
       out->gpu_launches += nl;
     } else {
       P.doc_map = S.d_map;
       for (int k = 0; k < 6; k++) {
         if (!cls_cnt[k]) continue;
         int nl = 0;
-        CK(launch_chat_translate_range(P, cls_start[k], cls_cnt[k], kClsMax[k], ctx->device, ctx->sm_count, ctx->s_compute, ctx->d_work, ctx->work_cap, &ctx->aux, &nl));
+        CK(launch_chat_translate_range(P, cls_start[k], cls_cnt[k], kClsMax[k], ctx->device, ctx->sm_count, ctx->s_compute, ctx->d_work, ctx->work_cap, &nl));
         out->gpu_launches += nl;
       }
     }
@@ -775,10 +747,6 @@ static int stream_chunks_core(aigw_ctx* ctx, uint32_t n, GET&& get, aigw_chunk_r
   if (arena) *arena = nullptr;
   if (n == 0) return 0;
   CK(cudaSetDevice(ctx->device));
-  static const bool prof = getenv("AIGW_STREAM_PROF") != nullptr;
-  auto now = [] { return std::chrono::steady_clock::now(); };
-  auto us = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double, std::micro>(b - a).count(); };
-  const auto t0 = now();
   ENSURE(sp.h_steps, sp.h_steps_cap, (size_t)n * sizeof(StreamStep), true);
   sp.call_no++;
   uint64_t in_bytes = 0, out_bytes = 0;
@@ -804,9 +772,7 @@ static int stream_chunks_core(aigw_ctx* ctx, uint32_t n, GET&& get, aigw_chunk_r
   ENSURE(sp.d_out, sp.d_out_cap, out_bytes + 16, false);
   ENSURE(sp.d_packed, sp.d_packed_cap, out_bytes + 16, false);
   if (!sp.d_used) { CK(cudaMalloc(&sp.d_used, 8)); CK(cudaHostAlloc(&sp.h_used, 8, cudaHostAllocDefault)); }
-  const auto t1 = now();
   if (!zc_base) host_parallel_for(n, [&](uint32_t b, uint32_t e) { for (uint32_t i = b; i < e; i++) { const StreamCallIn c = get(i); if (c.len) memcpy(sp.h_in + sp.h_steps[i].in_off, c.bytes, c.len); } });   // no caller pointer is retained
-  const auto t2 = now();
   cudaStream_t st = ctx->s_compute;
   if (!zc_base) CK(cudaMemcpyAsync(sp.d_in, sp.h_in, in_bytes, cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(sp.d_steps, sp.h_steps, (size_t)n * sizeof(StreamStep), cudaMemcpyHostToDevice, st));
@@ -820,18 +786,15 @@ static int stream_chunks_core(aigw_ctx* ctx, uint32_t n, GET&& get, aigw_chunk_r
   CK(cudaMemcpyAsync(hres, sp.d_res, (size_t)n * sizeof(aigw_chunk_result), cudaMemcpyDeviceToHost, st));
   CK(cudaMemcpyAsync(sp.h_used, sp.d_used, 8, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
-  const auto t3 = now();
   const uint64_t used = *sp.h_used < sp.d_packed_cap ? *sp.h_used : sp.d_packed_cap;
   if (used) {
     ENSURE(sp.h_packed, sp.h_packed_cap, used + 16, true);
     CK(cudaMemcpyAsync(sp.h_packed, sp.d_packed, used, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
   }
-  const auto t4 = now();
   if (res_pinned) { for (uint32_t i = 0; i < n; i++) sp.carry[sp.h_steps[i].slot] = results[i].carry_len; }
   else host_parallel_for(n, [&](uint32_t b, uint32_t e) { for (uint32_t i = b; i < e; i++) { results[i] = sp.h_res[i]; sp.carry[sp.h_steps[i].slot] = sp.h_res[i].carry_len; } });   // a stream appears once per call: the carry writes are disjoint
   if (arena) *arena = sp.h_packed;
-  if (prof && (sp.call_no & 63) == 1) fprintf(stderr, "stream_chunks n=%u%s: table %.0f us, byte staging %.0f us, H2D + kernels + D2H results %.0f us, D2H packed %.0f us, result copy %.0f us\n", n, zc_base ? " (zero-copy input)" : "", us(t0, t1), us(t1, t2), us(t2, t3), us(t3, t4), us(t4, now()));
   return 0;
 }
 }  // extern "C++"
@@ -846,9 +809,8 @@ int aigw_stream_chunks_soa(aigw_ctx* ctx, const uint64_t* handles, const uint8_t
   std::lock_guard<std::mutex> lk(ctx->sp.mu);
   const uint8_t* zc_dev = nullptr;
   {
-    static const bool no_zc = getenv("AIGW_STREAM_NO_ZEROCOPY") != nullptr;
     cudaPointerAttributes at;
-    if (!no_zc && base && cudaPointerGetAttributes(&at, base) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer) zc_dev = (const uint8_t*)at.devicePointer;
+    if (base && cudaPointerGetAttributes(&at, base) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer) zc_dev = (const uint8_t*)at.devicePointer;
     else cudaGetLastError();
   }
   return stream_chunks_core(ctx, n, [&](uint32_t i) { return StreamCallIn{handles[i], base + off[i], len[i], eos ? (uint32_t)eos[i] : 0u}; }, results, arena, zc_dev ? base : nullptr, zc_dev);

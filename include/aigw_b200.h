@@ -173,10 +173,9 @@ int aigw_chat_translate_device(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const
 int aigw_chat_translate_device_mapped(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const uint8_t* d_bodies, const uint64_t* d_offsets, const uint32_t* d_lens,
                                       const uint32_t* d_doc_map, uint32_t first, uint32_t count, uint32_t max_len, uint8_t* d_out, uint64_t out_capacity,
                                       aigw_doc_result* d_results, uint64_t* d_out_used, void* stream, float* kernel_ms);
-/* Stage profiling.  A device call normally splits its documents into L2-sized sub-batches that alternate between two internal
- * streams (the walk of one runs under the index / emit of the other), so per-stage times do not exist.  After
- * aigw_chat_set_profile(ctx, 1), calls that pass kernel_ms != NULL run the stages back to back on one stream and
- * aigw_chat_last_profile returns their CUDA-event times (index, walk, emit) and the launch count of the last call. */
+/* Stage profiling.  A device call runs its documents in sub-batches of up to 256 Ki documents, the stages of each back to back
+ * on the call's stream.  After aigw_chat_set_profile(ctx, 1), calls that pass kernel_ms != NULL also record CUDA events
+ * between the stages, and aigw_chat_last_profile returns their times (index, walk, emit) and the launch count of the last call. */
 int aigw_chat_set_profile(aigw_ctx* ctx, int on);
 int aigw_chat_last_profile(aigw_ctx* ctx, float stage_ms[3], int* launches);
 
@@ -197,7 +196,7 @@ int aigw_chat_translate_host(aigw_ctx* ctx, const aigw_backend_cfg* cfg, const u
 /* Calls of at most max_docs bodies whose largest body fits the 5120-byte class run as ONE fused kernel (index + walk + emit of
  * one document per CTA, bodies read in place from a mapped pinned buffer, records stored straight into the pinned output):
  * this is the latency path of a single request (ext_proc's per-request call, processor_impl.go:211-295) and of a batching
- * window.  Default 512 (AIGW_SMALL_MAX overrides); 0 sends every call through the throughput pipeline; -1 restores the default.
+ * window.  Default 512; 0 sends every call through the throughput pipeline; -1 restores the default.
  * Both paths produce the same bytes (same stage code). */
 void aigw_chat_set_small_batch(aigw_ctx* ctx, int max_docs);
 
